@@ -1,8 +1,12 @@
 #!/usr/bin/env python
 """bench.py -- ECDSA-P256 verifies/sec of the B200 verifier (BASELINE.json metric) and of the reference's CPU path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch B] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step of `value` returned -- the all-gathered validity bitmask, one float32 0/1
+per signature in the order that step verified them -- as DIR/valid.npy.  The inputs are seeded, so two builds run with the
+same arguments can be compared output for output.
 
 A "step" is one pass of the hot path over one batch of B synthetic signatures per GPU (default B = 65 536, the
 BASELINE.json configs[1] workload: K = 64 keys, SHA-256 digests of 1 KiB messages, low-S DER signatures).  With N > 1
@@ -269,7 +273,7 @@ def run_gpu(args):
     for k in range(args.warmup):
         full = step(k)
     sync_all()
-    assert bool((full == -1).all()), "warm-up bitmask is not all-valid"
+    assert args.warmup == 0 or bool((full == -1).all()), "warm-up bitmask is not all-valid"
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -286,6 +290,8 @@ def run_gpu(args):
     launches = ctx.launch_count() - launches0
     dev_ms = sum(a.elapsed_time(b) for a, b in ev)
     assert bool((full == -1).all())
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"valid": np.unpackbits(full.cpu().numpy().view(np.uint8), bitorder="little")[:n_total]})
     # the same loop with the L2 overwritten between steps (256 MiB fill, outside the event pairs)
     fev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(args.steps)]
     sync_all()
@@ -703,7 +709,12 @@ def main():
     ap.add_argument("--no-parity", action="store_true", help="skip the (untimed) named-shape parity leg")
     ap.add_argument("--no-clients", action="store_true", help="skip the block-replay variant with 2 000 client identities")
     ap.add_argument("--collective", default="nccl", choices=["p2p", "nccl"], help="N > 1: how the bitmask is reassembled in the timed loop (the other way is timed beside it)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the validity bits of the last timed step to DIR/valid.npy (GPU arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     # The contract is ONE JSON line on stdout.  Libraries write there too (NCCL prints its version line on the first
     # collective), so everything but the result goes to stderr: fd 1 is pointed at fd 2 for the duration of the run and the
     # JSON line is written to the saved descriptor.
@@ -719,6 +730,19 @@ def main():
 
 
 _RESULT_FD = None
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(dirname, arrays):
+    """Writes each array as DIR/<name>.npy in float32.  Past 64 MB in all, each keeps a fixed, seeded sample of its entries (in
+    their original order), so runs with the same arguments still write the same sample."""
+    os.makedirs(dirname, exist_ok=True)
+    cap = (DUMP_BYTES // len(arrays) - 4096) // 4                        # entries per array; 4096 B leaves room for the .npy header
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float32).reshape(-1)
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
 
 
 def emit(obj):

@@ -32,6 +32,21 @@ def test_reference_arm_other_ranks_are_silent():
     assert _run({"RANK": "1", "WORLD_SIZE": "2", "LOCAL_RANK": "1"}).strip() == ""
 
 
+def test_dump_outputs_writes_float32_and_samples_past_the_cap(tmp_path, monkeypatch):
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    bits = np.unpackbits(np.arange(256, dtype=np.uint8))
+    bench.dump_outputs(str(tmp_path / "full"), {"valid": bits})
+    got = np.load(str(tmp_path / "full" / "valid.npy"))
+    assert got.dtype == np.float32 and (got == bits).all()
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 4 * 100)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), {"valid": np.arange(1000)})
+    a, b = (np.load(str(tmp_path / d / "valid.npy")) for d in ("a", "b"))
+    assert a.dtype == np.float32 and a.size == 100 and (a == b).all() and (np.diff(a) > 0).all()
+
+
 def test_alg_mac_model_matches_the_window_shapes():
     sys.path.insert(0, ROOT)
     import bench
