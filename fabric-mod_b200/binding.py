@@ -11,6 +11,8 @@ LIB_PATH = os.environ.get("FABGPU_LIB") or os.path.join(_HERE, "lib", "libfabgpu
 SLOTS = 3
 
 OK, E_NO_DEVICE, E_CUDA, E_ARG, E_INJECTED = 0, -1, -2, -3, -4
+HASH_SHA2, HASH_SHA3 = 0, 1          # FABGPU_HASH_*: the SignatureHashFamily of an MSP
+HASH_FAMILIES = {"SHA2": HASH_SHA2, "SHA3": HASH_SHA3}
 (ST_VALID, ST_INVALID, ST_ERR_NIL_KEY, ST_ERR_EMPTY_SIG, ST_ERR_EMPTY_DIGEST, ST_ERR_UNMARSHAL, ST_ERR_R_NOT_POSITIVE,
  ST_ERR_S_NOT_POSITIVE, ST_ERR_HIGH_S, ST_ERR_UNSUPPORTED_KEY, ST_ERR_OFF_CURVE) = range(11)
 
@@ -24,7 +26,7 @@ EXPORTS = [
     "fabgpu_verify_p256_keyed_async", "fabgpu_verify_p256_device_keyed", "fabgpu_last_timing", "fabgpu_build_info",
     "fabgpu_msp_configure", "fabgpu_validate_block", "fabgpu_validate_envelopes", "fabgpu_block_buffer", "fabgpu_block_timing", "fabgpu_sha256_segments",
     "fabgpu_bccsp_verify_batch_async", "fabgpu_bccsp_verify_batch_wait", "fabgpu_bccsp_batch_buffers", "fabgpu_bccsp_verify_batch_inplace_async",
-    "fabgpu_msp_identity_groups", "fabgpu_namespace_policies",
+    "fabgpu_msp_identity_groups", "fabgpu_namespace_policies", "fabgpu_msp_hash_families", "fabgpu_sha3_256_segments",
     "fabgpu_peer_mask_create", "fabgpu_peer_mask_open", "fabgpu_peer_mask_close", "fabgpu_verify_p256_device_keyed_allgather",
     "fabgpu_validate_block_async", "fabgpu_validate_envelopes_async", "fabgpu_validate_wait", "fabgpu_block_buffer_slot",
     "fabgpu_keys_register_small", "fabgpu_small_slot_capacity", "fabgpu_key_table_stats", "fabgpu_small_table_info",
@@ -362,10 +364,12 @@ class Context:
         return bool(valid.value), (e if e else None)
 
     # ---- block level ------------------------------------------------------------------------------------
-    def msp_configure(self, identities, policy_nodes, principals, channel, policies=None):
+    def msp_configure(self, identities, policy_nodes, principals, channel, policies=None, hash_families=None):
         """identities: list of (serialized: bytes, mspid: str, key_xy: 64 bytes, valid: bool).  policy_nodes may hold several policy
         trees; policies = {namespace: root node index} names the tree of each chaincode namespace (None: node 0 for every namespace).
-        The identities' de-duplication groups (Mspid + certificate, identity_groups) are installed as well."""
+        The identities' de-duplication groups (Mspid + certificate, identity_groups) are installed as well.
+        hash_families = {mspid: "SHA2" | "SHA3"}: the SignatureHashFamily of those MSPs (fabgpu_msp_hash_families); None or an MSP
+        left out: SHA2."""
         def blob(items):
             off = np.zeros(len(items) + 1, np.uint32)
             off[1:] = np.cumsum([len(x) for x in items])
@@ -387,6 +391,20 @@ class Context:
         nb, no = blob([n.encode() for n in names])
         roots = np.array([policies[n] for n in names] or [0], np.int32)
         self._ck(lib().fabgpu_namespace_policies(self._h, _p(nb), _p(no), _p(roots), ctypes.c_int(len(names))))
+        if hash_families is not None:
+            self.msp_hash_families(hash_families)
+
+    def msp_hash_families(self, hash_families):
+        """{mspid: "SHA2" | "SHA3"} -> fabgpu_msp_hash_families (after msp_configure; {} restores all-SHA2)."""
+        unknown = {f for f in hash_families.values() if f not in HASH_FAMILIES}
+        if unknown:
+            raise ValueError("hash family must be SHA2 or SHA3, got %s" % sorted(map(str, unknown)))
+        names = sorted(hash_families)
+        off = np.zeros(len(names) + 1, np.uint32)
+        off[1:] = np.cumsum([len(n.encode()) for n in names])
+        mb = np.ascontiguousarray(np.frombuffer(b"".join(n.encode() for n in names) or b"\x00", np.uint8))
+        fam = np.array([HASH_FAMILIES[hash_families[n]] for n in names] or [0], np.uint8)
+        self._ck(lib().fabgpu_msp_hash_families(self._h, _p(mb), _p(off), _p(fam), ctypes.c_int(len(names))))
 
     def block_buffer(self, nbytes, slot=0):
         """Pinned staging buffer (numpy view) for block bytes; one per slot."""
@@ -452,6 +470,14 @@ class Context:
         jobs = np.ascontiguousarray(jobs, dtype=np.uint32).reshape(-1, 6)
         out = np.zeros((jobs.shape[0], 32), np.uint8)
         self._ck(lib().fabgpu_sha256_segments(self._h, _p(buf), ctypes.c_size_t(buf.shape[0]), _p(jobs), ctypes.c_size_t(jobs.shape[0]), _p(out)))
+        return out
+
+    def sha3_256_segments(self, buf, jobs):
+        """jobs: uint32[n,6] (off0,off1,off2,len0,len1,len2) -> uint8[n,32] SHA3-256 digests."""
+        buf = np.ascontiguousarray(np.frombuffer(buf, np.uint8) if isinstance(buf, (bytes, bytearray)) else buf)
+        jobs = np.ascontiguousarray(jobs, dtype=np.uint32).reshape(-1, 6)
+        out = np.zeros((jobs.shape[0], 32), np.uint8)
+        self._ck(lib().fabgpu_sha3_256_segments(self._h, _p(buf), ctypes.c_size_t(buf.shape[0]), _p(jobs), ctypes.c_size_t(jobs.shape[0]), _p(out)))
         return out
 
     def last_timing(self):

@@ -46,6 +46,8 @@ struct MspDev {
     const int32_t* group;         // per identity: de-duplication id -- Mspid + certificate (policy.go:380-386): two serializations of one
                                   // certificate share it; null = every table entry is its own group
     const uint8_t* keys_xy;       // per identity: X || Y (64 bytes), for signatures whose key has no table
+    const uint8_t* hash_kind = nullptr;   // per identity: hash of identity.Verify, 0 = SHA-256, 1 = SHA3-256 (the MSP's SignatureHashFamily,
+                                          // msp/identities.go:169-196,216-224); null = SHA-256 for every identity
     const uint64_t* ht_hash;      // open-addressing table, size ht_size (power of two); 0 = empty
     const int32_t* ht_idx;
     uint32_t ht_size;
@@ -292,6 +294,7 @@ struct JobArrays {
     int32_t* identity;             // [J_cap]
     uint8_t* qx; uint8_t* qy;      // [J_cap x 32] or null: filled only for keys without a table (generic kernel)
     uint8_t* gate_ok;              // [J_cap]
+    uint8_t* kind = nullptr;       // [J_cap] or null: hash of each signature message, from its signer's MspDev::hash_kind
     uint32_t J_cap;                // capacity; creator jobs occupy [0, T), endorsement jobs [T, T + n_end)
     uint32_t T;
 };
@@ -511,6 +514,8 @@ BD_HD void resolve_job(const uint8_t* base, uint32_t j, const RawJob* raw, const
     }
     ja.gate_ok[j] = ok ? 1 : 0;
     ja.identity[j] = identity;
+    // creator jobs hash with the creator's MSP family, endorsement jobs with the endorser's: the identity that verifies the signature
+    if (ja.kind) ja.kind[j] = (identity >= 0 && msp.hash_kind) ? msp.hash_kind[identity] : 0;
     const int32_t slot = (identity >= 0 && ok) ? msp.key_slot[identity] : -1;
     ja.key_slot[j] = slot;
     if (identity >= 0 && ok && slot == -1 && ja.qx) {

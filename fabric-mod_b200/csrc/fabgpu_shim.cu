@@ -23,6 +23,7 @@
 #include "bccsp_host.hpp"
 #include "blockval.hpp"
 #include "sha256.cuh"
+#include "sha3.cuh"
 #include "blockdev_kernels.cuh"
 #include "ecdsa_kernels.cuh"
 
@@ -207,6 +208,7 @@ struct fabgpu_ctx {
         uint8_t* ns_blob = nullptr; uint32_t* ns_off = nullptr; int32_t* ns_root = nullptr; int32_t n_ns = 0;    // fabgpu_namespace_policies
         uint64_t* ht_hash = nullptr; uint32_t ht_size = 0; int32_t n_ids = 0, n_nodes = 0, n_principals = 0; uint32_t channel_len = 0;
         bool all_slots = true; int classes = 0;                    // which non-big classes the identities' keys fall in (CLASS_*)
+        uint8_t* hash_kind = nullptr; bool any_sha3 = false;        // per identity: SHA_KIND_* of its MSP (fabgpu_msp_hash_families)
     } dm;
     struct GateBufs {                          // fabgpu_bccsp_verify_batch with device-side gates
         size_t n_cap = 0, sig_cap = 0, dig_cap = 0, k_cap = 0;
@@ -226,6 +228,7 @@ struct fabgpu_ctx {
         uint32_t* d_env_off = nullptr; bdev::TxDev* d_txs = nullptr; bdev::RawJob* d_raw = nullptr; bdev::ShaJobD* d_sha = nullptr; uint8_t *d_r = nullptr, *d_s = nullptr, *d_qx = nullptr,
         *d_qy = nullptr, *d_gate = nullptr, *d_dig = nullptr, *d_flags = nullptr; int32_t *d_ks = nullptr, *d_ident = nullptr; uint32_t *d_mask = nullptr,
         *d_off = nullptr, *d_counter = nullptr, *d_idx = nullptr; uint64_t* d_hash = nullptr; bdev::Seg* d_seg = nullptr;
+        uint8_t* d_kind = nullptr;               // per signature job: SHA_KIND_* (written only when the MSP table holds a SHA3 identity)
         uint8_t* h_flags = nullptr; uint64_t* h_hash = nullptr; bdev::Seg* h_seg = nullptr; uint32_t* h_counter = nullptr; uint32_t* h_env_off = nullptr;
         // the block in flight on this slot (fabgpu_validate_*_async .. fabgpu_validate_wait)
         bool busy = false, on_device = false, use_ev = false; size_t T = 0; const uint8_t* block = nullptr;
@@ -494,11 +497,11 @@ void free_all(fabgpu_ctx* ctx)
         }
         auto& dm = ctx->dm;
         void* dev2[] = {dm.id_blob, dm.valid, dm.keys_xy, dm.channel, dm.id_off, dm.key_slot, dm.msp_code, dm.ht_idx, dm.nodes, dm.principal_code, dm.ht_hash,
-                        dm.group, dm.ns_blob, dm.ns_off, dm.ns_root};
+                        dm.group, dm.ns_blob, dm.ns_off, dm.ns_root, dm.hash_kind};
         for (void* p : dev2) if (p) cudaFree(p);
         for (auto& db : ctx->dbs) {
             void* dev4[] = {db.d_env_off, db.d_txs, db.d_raw, db.d_sha, db.d_r, db.d_s, db.d_qx, db.d_qy, db.d_gate, db.d_dig, db.d_flags, db.d_ks, db.d_ident, db.d_mask, db.d_off,
-                            db.d_counter, db.d_hash, db.d_seg, db.d_idx};
+                            db.d_counter, db.d_hash, db.d_seg, db.d_idx, db.d_kind};
             for (void* p : dev4) if (p) cudaFree(p);
             void* host2[] = {db.h_flags, db.h_hash, db.h_seg, db.h_counter, db.h_env_off};
             for (void* p : host2) if (p) cudaFreeHost(p);
@@ -1670,7 +1673,7 @@ static int upload_msp(fabgpu_ctx* ctx, const uint8_t* id_blob, const uint32_t* i
     // blocks already enqueued on a slot were launched with the OLD tables (passed by value): let them finish before those go away
     for (auto& ds : ctx->devs[0].slot) CK(ctx, cudaStreamSynchronize(ds.stream));
     void* old[] = {dm.id_blob, dm.valid, dm.keys_xy, dm.channel, dm.id_off, dm.key_slot, dm.msp_code, dm.ht_idx, dm.nodes, dm.principal_code, dm.ht_hash,
-                   dm.group, dm.ns_blob, dm.ns_off, dm.ns_root};
+                   dm.group, dm.ns_blob, dm.ns_off, dm.ns_root, dm.hash_kind};
     for (void* p : old) if (p) cudaFree(p);
     dm = fabgpu_ctx::DevMsp();
     // MSP-id codes: equal strings <=> equal codes, shared between identities and policy principals
@@ -1715,6 +1718,8 @@ static int upload_msp(fabgpu_ctx* ctx, const uint8_t* id_blob, const uint32_t* i
     rc |= up(dm.nodes, policy_nodes, 16 * (size_t)n_nodes);
     rc |= up(dm.principal_code, pcode.data(), 4 * ctx->principals.size());
     rc |= up(dm.channel, ctx->channel.data(), ctx->channel.size());
+    const std::vector<uint8_t> sha2(n_ids > 0 ? n_ids : 1, SHA_KIND_SHA2);      // every identity SHA-256 until fabgpu_msp_hash_families
+    rc |= up(dm.hash_kind, sha2.data(), (size_t)n_ids);
     if (rc) return FABGPU_E_CUDA;
     dm.ht_size = n_ids ? hsz : 0; dm.n_ids = n_ids; dm.n_nodes = n_nodes; dm.n_principals = (int32_t)ctx->principals.size();
     dm.channel_len = (uint32_t)ctx->channel.size();
@@ -1826,6 +1831,39 @@ int fabgpu_namespace_policies(fabgpu_ctx* ctx, const uint8_t* ns_blob, const uin
     return FABGPU_OK;
 }
 
+int fabgpu_msp_hash_families(fabgpu_ctx* ctx, const uint8_t* mspid_blob, const uint32_t* mspid_off, const uint8_t* family, int n_msps)
+{
+    if (!ctx || n_msps < 0 || (n_msps && (!mspid_blob || !mspid_off || !family))) return FABGPU_E_ARG;
+    std::lock_guard<std::mutex> lk0(ctx->slot0_mu);
+    auto& dm = ctx->dm;
+    std::unordered_map<std::string, uint8_t> fam;
+    for (int i = 0; i < n_msps; i++) {
+        const std::string id((const char*)mspid_blob + mspid_off[i], mspid_off[i + 1] - mspid_off[i]);
+        if (family[i] != FABGPU_HASH_SHA2 && family[i] != FABGPU_HASH_SHA3) {
+            ctx->last_error = "hash family of MSP '" + id + "' is neither FABGPU_HASH_SHA2 nor FABGPU_HASH_SHA3"; return FABGPU_E_ARG;
+        }
+        auto it = fam.find(id);
+        if (it != fam.end() && it->second != family[i]) { ctx->last_error = "MSP '" + id + "' is listed with two hash families"; return FABGPU_E_ARG; }
+        fam[id] = family[i];
+    }
+    for (const auto& kv : fam) {
+        bool carried = false;
+        for (const auto& m : ctx->msp.mspid) if (m == kv.first) { carried = true; break; }
+        if (!carried) { ctx->last_error = "no identity of the MSP table belongs to MSP '" + kv.first + "'"; return FABGPU_E_ARG; }
+    }
+    const int n_ids = dm.n_ids;
+    std::vector<uint8_t> kind(n_ids > 0 ? n_ids : 1, SHA_KIND_SHA2);
+    bool any = false;
+    for (int i = 0; i < n_ids; i++) {
+        auto it = fam.find(ctx->msp.mspid[i]);
+        if (it != fam.end() && it->second == FABGPU_HASH_SHA3) { kind[i] = SHA_KIND_SHA3; any = true; }
+    }
+    int rc = drain_block_streams(ctx); if (rc) return rc;
+    if (n_ids) CK(ctx, cudaMemcpy(dm.hash_kind, kind.data(), (size_t)n_ids, cudaMemcpyHostToDevice));
+    dm.any_sha3 = any;
+    return FABGPU_OK;
+}
+
 int fabgpu_block_buffer_slot(fabgpu_ctx* ctx, int slot, size_t bytes, uint8_t** out)
 {
     if (!ctx || !out || slot < 0 || slot >= FABGPU_SLOTS) return FABGPU_E_ARG;
@@ -1843,7 +1881,8 @@ int fabgpu_block_buffer(fabgpu_ctx* ctx, size_t bytes, uint8_t** out) { return f
 
 // Device path of the block pre-pass: the host only copies bytes in and flags out (and marks duplicate tx ids).
 //   H2D block + envelope offsets -> block_walk_kernel (per transaction) -> block_resolve_kernel (per signature: identity lookup, DER gates)
-//   -> sha256_segments_kernel (signed messages + check digests) -> one verify launch -> block_decide_kernel -> D2H flags.
+//   -> sha256_segments_kernel (signed messages + check digests; sha3_256_segments_kernel beside it for the signed messages of SHA3 MSPs)
+//   -> one verify launch -> block_decide_kernel -> D2H flags.
 // Everything is enqueued on the slot's stream in one go: the number of endorsement jobs (known only after the walk) stays
 // on the device -- the later launches are sized for the worst case and read the count themselves.
 static int block_submit(fabgpu_ctx* ctx, int slot, const uint8_t* block, size_t block_len, const uint32_t* env_off, size_t n_env)
@@ -1918,7 +1957,7 @@ static int block_submit(fabgpu_ctx* ctx, int slot, const uint8_t* block, size_t 
         rc |= grow_dev(ctx, db.d_raw, sizeof(bdev::RawJob) * jc);
         rc |= grow_dev(ctx, db.d_sha, sizeof(bdev::ShaJobD) * (jc + 2 * tc)); rc |= grow_dev(ctx, db.d_dig, 32 * (jc + 2 * tc) + 64);
         rc |= grow_dev(ctx, db.d_r, 32 * jc); rc |= grow_dev(ctx, db.d_s, 32 * jc); rc |= grow_dev(ctx, db.d_qx, 32 * jc); rc |= grow_dev(ctx, db.d_qy, 32 * jc);
-        rc |= grow_dev(ctx, db.d_gate, jc); rc |= grow_dev(ctx, db.d_ks, 4 * jc); rc |= grow_dev(ctx, db.d_ident, 4 * jc);
+        rc |= grow_dev(ctx, db.d_gate, jc); rc |= grow_dev(ctx, db.d_ks, 4 * jc); rc |= grow_dev(ctx, db.d_ident, 4 * jc); rc |= grow_dev(ctx, db.d_kind, jc);
         rc |= grow_dev(ctx, db.d_mask, jc / 8 + 8); rc |= grow_dev(ctx, db.d_off, jc / 8 + 8); rc |= grow_dev(ctx, db.d_counter, 16); rc |= grow_dev(ctx, db.d_idx, 4 * (jc + 2));
         rc |= grow_dev(ctx, db.d_flags, tc); rc |= grow_dev(ctx, db.d_hash, 8 * tc); rc |= grow_dev(ctx, db.d_seg, 8 * tc);
         rc |= grow_host(ctx, db.h_flags, tc); rc |= grow_host(ctx, db.h_hash, 8 * tc); rc |= grow_host(ctx, db.h_seg, 8 * tc);
@@ -1935,12 +1974,17 @@ static int block_submit(fabgpu_ctx* ctx, int slot, const uint8_t* block, size_t 
     CK(ctx, cudaMemcpyAsync(db.d_env_off, db.h_env_off, 8 * T, cudaMemcpyHostToDevice, st));
     CK(ctx, cudaMemsetAsync(db.d_counter, 0, 16, st));
     bdev::MspDev m; m.id_blob = dm.id_blob; m.id_off = dm.id_off; m.key_slot = dm.key_slot; m.valid = dm.valid; m.msp_code = dm.msp_code; m.group = dm.group;
-    m.keys_xy = dm.keys_xy; m.ht_hash = dm.ht_hash; m.ht_idx = dm.ht_idx; m.ht_size = dm.ht_size; m.n_ids = dm.n_ids;
+    m.keys_xy = dm.keys_xy; m.ht_hash = dm.ht_hash; m.ht_idx = dm.ht_idx; m.ht_size = dm.ht_size; m.n_ids = dm.n_ids; m.hash_kind = dm.hash_kind;
     bdev::PolicyDev pol; pol.nodes = dm.nodes; pol.n_nodes = dm.n_nodes; pol.principal_code = dm.principal_code; pol.n_principals = dm.n_principals;
     pol.ns_blob = dm.ns_blob; pol.ns_off = dm.ns_off; pol.ns_root = dm.ns_root; pol.n_ns = dm.n_ns;
     const bool need_q = (dm.classes & CLASS_GENERIC) != 0;   // only the generic arithmetic reads the key itself
     bdev::JobArrays ja; ja.sha = db.d_sha; ja.r = db.d_r; ja.s = db.d_s; ja.key_slot = db.d_ks; ja.identity = db.d_ident; ja.qx = need_q ? db.d_qx : nullptr;
     ja.qy = need_q ? db.d_qy : nullptr; ja.gate_ok = db.d_gate; ja.J_cap = (uint32_t)J_cap; ja.T = (uint32_t)T;
+    // An MSP with SignatureHashFamily SHA3 in the table: resolve writes each signature job's hash kind, the SHA-256 launches skip the
+    // SHA3 jobs and a SHA3-256 launch beside each hashes them into the same digest slots.  Otherwise the launches are those of a
+    // SHA-256-only table (kind = null).
+    const bool sha3 = dm.any_sha3;
+    ja.kind = sha3 ? db.d_kind : nullptr;
     const uint32_t cnt = (uint32_t)T, E_cap = (uint32_t)(J_cap - T);
     // One copy, then the walk.  (Copying in chunks with a walk per chunk was measured slower on B200 -- 1 chunk 1.93 ms, 4 chunks
     // 2.27 ms, 8 chunks 3.52 ms per 10k-tx block: hashing a 4.6 KB payload is ~250 us of dependent rounds per thread however few
@@ -1949,16 +1993,21 @@ static int block_submit(fabgpu_ctx* ctx, int slot, const uint8_t* block, size_t 
     CK(ctx, cudaMemcpyAsync(bb.d_block, block, block_len, cudaMemcpyHostToDevice, st));
     bdev::block_walk_kernel<<<(cnt + 31) / 32, 32, 0, st>>>(bb.d_block, db.d_env_off, 0u, cnt, cnt, dm.channel, dm.channel_len, db.d_txs, db.d_raw, ja, db.d_counter);
     bdev::block_resolve_kernel<<<(cnt + 63) / 64, 64, 0, st>>>(bb.d_block, db.d_raw, 0u, cnt, m, ja, db.d_txs);                      // creator jobs
-    sha256_segments_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha), cnt, db.d_dig);
+    sha256_segments_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha), cnt, db.d_dig, nullptr, ja.kind);
+    if (sha3) sha3_256_segments_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha), cnt, db.d_dig, nullptr, ja.kind);
+    // tx id and proposal hash: SHA-256 whatever the MSP family (protoutil/proputils.go:355-364, protoutil/txutils.go:431-448)
     sha256_segments_kernel<<<(2 * cnt + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha + J_cap), 2 * cnt, db.d_dig + 32 * J_cap);
-    ctx->launches += 4;
+    ctx->launches += sha3 ? 5 : 4;
     CK(ctx, cudaGetLastError());
     if (db.use_ev) CK(ctx, cudaEventRecord(db.ev[1], st));
     if (db.use_ev) CK(ctx, cudaEventRecord(db.ev[2], st));
     // endorsement jobs [T, T + *d_counter): launches sized for the worst case, the kernels stop at the device-side count
     bdev::block_resolve_kernel<<<(E_cap + 63) / 64, 64, 0, st>>>(bb.d_block, db.d_raw, cnt, E_cap, m, ja, db.d_txs, db.d_counter);
-    sha256_segments_kernel<<<(E_cap + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha) + T, E_cap, db.d_dig + 32 * T, db.d_counter);
-    ctx->launches += 2;
+    sha256_segments_kernel<<<(E_cap + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha) + T, E_cap, db.d_dig + 32 * T, db.d_counter,
+                                                               sha3 ? ja.kind + T : nullptr);
+    if (sha3) sha3_256_segments_kernel<<<(E_cap + 127) / 128, 128, 0, st>>>(bb.d_block, reinterpret_cast<const ShaJob*>(db.d_sha) + T, E_cap, db.d_dig + 32 * T,
+                                                                            db.d_counter, ja.kind + T);
+    ctx->launches += sha3 ? 3 : 2;
     CK(ctx, cudaGetLastError());
     if (db.use_ev) CK(ctx, cudaEventRecord(db.ev[3], st));
     int rc = launch_verify(ctx, dv, dm.all_slots ? MODE_CACHED : MODE_MIXED, db.d_ks, db.d_qx, db.d_qy, db.d_dig, db.d_r, db.d_s, J_cap, db.d_mask, db.d_off, st,
@@ -2122,6 +2171,28 @@ int fabgpu_sha256_segments(fabgpu_ctx* ctx, const uint8_t* buf, size_t buf_len, 
     CK(ctx, cudaMemcpy(d_jobs, jobs, sizeof(ShaJob) * n, cudaMemcpyHostToDevice));
     if (n) {
         sha256_segments_kernel<<<(unsigned)((n + 127) / 128), 128>>>(d_buf, d_jobs, (uint32_t)n, d_dig);
+        ctx->launches++;
+        CK(ctx, cudaGetLastError());
+    }
+    CK(ctx, cudaMemcpy(digests, d_dig, 32 * n, cudaMemcpyDeviceToHost));
+    cudaFree(d_buf); cudaFree(d_jobs); cudaFree(d_dig);
+    return FABGPU_OK;
+}
+
+// digests[j] = SHA3-256(buf[off0..) || buf[off1..) || buf[off2..)) on the device; same job layout as fabgpu_sha256_segments
+int fabgpu_sha3_256_segments(fabgpu_ctx* ctx, const uint8_t* buf, size_t buf_len, const uint32_t* jobs, size_t n, uint8_t* digests)
+{
+    if (!ctx || !buf || !jobs || !digests) return FABGPU_E_ARG;
+    std::lock_guard<std::mutex> lk0(ctx->slot0_mu);
+    Device& dv = ctx->devs[0];
+    CK(ctx, cudaSetDevice(dv.id));
+    uint8_t *d_buf = nullptr, *d_dig = nullptr; ShaJob* d_jobs = nullptr;
+    // slack: the block loader reads the aligned word past a range's end
+    CK(ctx, cudaMalloc(&d_buf, buf_len + 8)); CK(ctx, cudaMalloc(&d_jobs, sizeof(ShaJob) * (n ? n : 1))); CK(ctx, cudaMalloc(&d_dig, 32 * (n ? n : 1)));
+    CK(ctx, cudaMemcpy(d_buf, buf, buf_len, cudaMemcpyHostToDevice));
+    CK(ctx, cudaMemcpy(d_jobs, jobs, sizeof(ShaJob) * n, cudaMemcpyHostToDevice));
+    if (n) {
+        sha3_256_segments_kernel<<<(unsigned)((n + 127) / 128), 128>>>(d_buf, d_jobs, (uint32_t)n, d_dig);
         ctx->launches++;
         CK(ctx, cudaGetLastError());
     }

@@ -15,6 +15,9 @@ namespace fabgpu {
 
 struct ShaJob { uint32_t off[3]; uint32_t len[3]; };
 
+// Hash of a signed message on the block path (bdev::JobArrays::kind): the SignatureHashFamily of the signer's MSP.
+enum : uint8_t { SHA_KIND_SHA2 = 0, SHA_KIND_SHA3 = 1 };
+
 __device__ __constant__ uint32_t kSha256K[64] = {
     0x428a2f98, 0x71374491, 0xb5c0fbcf, 0xe9b5dba5, 0x3956c25b, 0x59f111f1, 0x923f82a4, 0xab1c5ed5, 0xd807aa98, 0x12835b01, 0x243185be,
     0x550c7dc3, 0x72be5d74, 0x80deb1fe, 0x9bdc06a7, 0xc19bf174, 0xe49b69c1, 0xefbe4786, 0x0fc19dc6, 0x240ca1cc, 0x2de92c6f, 0x4a7484aa,
@@ -68,13 +71,15 @@ __device__ __forceinline__ uint32_t sha_msg_byte(const uint8_t* __restrict__ buf
 // (issued together) and re-aligned with funnel shifts, whatever the byte offset of the range; blocks that straddle two
 // ranges or contain padding are assembled byte by byte (at most three or four per message).
 // `buf` must be readable 4 bytes past the last range (the block buffer is allocated with slack).
+// kind != null: the jobs with kind[j] == SHA_KIND_SHA3 are skipped (sha3_256_segments_kernel hashes those).
 __global__ void __launch_bounds__(128)
 sha256_segments_kernel(const uint8_t* __restrict__ buf, const ShaJob* __restrict__ jobs, uint32_t n, uint8_t* __restrict__ digests,
-                       const uint32_t* __restrict__ n_dev = nullptr)
+                       const uint32_t* __restrict__ n_dev = nullptr, const uint8_t* __restrict__ kind = nullptr)
 {
     if (n_dev) n = min(n, *n_dev);               // message count produced by an earlier kernel of the stream; n is the launch bound
     const uint32_t j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j >= n) return;
+    if (kind && kind[j] == SHA_KIND_SHA3) return;
     const ShaJob job = jobs[j];
     uint32_t h[8] = {0x6a09e667, 0xbb67ae85, 0x3c6ef372, 0xa54ff53a, 0x510e527f, 0x9b05688c, 0x1f83d9ab, 0x5be0cd19};
     const uint64_t total = (uint64_t)job.len[0] + job.len[1] + job.len[2];

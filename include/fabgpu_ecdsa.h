@@ -235,6 +235,17 @@ int fabgpu_msp_configure(fabgpu_ctx* ctx, const uint8_t* id_blob, const uint32_t
  *       entry is flagged 254 (NOT_VALIDATED): the CPU validator reads the chaincode definition from the ledger. */
 int fabgpu_msp_identity_groups(fabgpu_ctx* ctx, const int32_t* group, int n_ids);
 int fabgpu_namespace_policies(fabgpu_ctx* ctx, const uint8_t* ns_blob, const uint32_t* ns_off, const int32_t* ns_root, int n_ns);
+/* A third refinement, called the same way: the hash each MSP's identities sign with.  identity.Verify hashes the signed message
+ * with the SignatureHashFamily of the signer's MSP configuration (FabricMSPConfig.CryptoConfig.SignatureHashFamily;
+ * msp/identities.go:169-196,216-224): "SHA2" -> SHA-256, "SHA3" -> SHA3-256.  family[i] (FABGPU_HASH_SHA2 or FABGPU_HASH_SHA3)
+ * is the family of MSP i (mspid_blob + (n_msps+1) offsets); each creator signature is hashed with the creator's family, each
+ * endorsement signature with the endorser's.  MSPs not listed stay SHA2; n_msps = 0 restores all-SHA2, and so does every
+ * fabgpu_msp_configure.  The tx-id check (protoutil/proputils.go:355-364) and the proposal hash (protoutil/txutils.go:431-448)
+ * are SHA-256 whatever the family.  FABGPU_E_ARG (with fabgpu_last_error) for a family code other than the two, an MSP id
+ * that no identity of the table carries, or one MSP listed twice with different families. */
+#define FABGPU_HASH_SHA2 0
+#define FABGPU_HASH_SHA3 1
+int fabgpu_msp_hash_families(fabgpu_ctx* ctx, const uint8_t* mspid_blob, const uint32_t* mspid_off, const uint8_t* family, int n_msps);
 /* flags[i] receives the validation code of transaction i; *n_tx_out the number of transactions. */
 int fabgpu_validate_block(fabgpu_ctx* ctx, const uint8_t* block, size_t block_len, uint8_t* flags, size_t flags_cap, size_t* n_tx_out);
 /* Same for a caller that already holds Block.Data.Data as separate byte strings (the Go validator does): `blob` is their
@@ -255,11 +266,14 @@ int fabgpu_block_buffer(fabgpu_ctx* ctx, size_t bytes, uint8_t** out);          
 int fabgpu_block_buffer_slot(fabgpu_ctx* ctx, int slot, size_t bytes, uint8_t** out);
 /* Times of the last completed block, microseconds.  [0..4] host wall clock: enqueue, (unused), wait for the device,
  * duplicate-tx-id pass, total from submit to flags.  [5..9] CUDA-event times of the device stages (FABGPU_BLOCK_EVENTS=1):
- * H2D + walk + creator resolve + SHA-256, (unused), endorsement resolve + SHA-256, verify kernel(s), block_decide_kernel. */
+ * H2D + walk + creator resolve + SHA-256, (unused), endorsement resolve + SHA-256, verify kernel(s), block_decide_kernel.
+ * (With a SHA3 MSP in the table the hash stages include the SHA3-256 launches.) */
 int fabgpu_block_timing(const fabgpu_ctx* ctx, double out_us[10]);
 /* Device SHA-256 of messages given as up to three byte ranges of `buf` each: jobs = n x {off0,off1,off2,len0,len1,len2}
  * (uint32); digests = n x 32 bytes.  (The hash msp identity.Verify computes first: msp/identities.go:178.) */
 int fabgpu_sha256_segments(fabgpu_ctx* ctx, const uint8_t* buf, size_t buf_len, const uint32_t* jobs, size_t n, uint8_t* digests);
+/* The same for SHA3-256 (FIPS 202), the digest of identity.Verify for an MSP whose SignatureHashFamily is SHA3. */
+int fabgpu_sha3_256_segments(fabgpu_ctx* ctx, const uint8_t* buf, size_t buf_len, const uint32_t* jobs, size_t n, uint8_t* digests);
 
 /* ---- test / bring-up hooks ------------------------------------------------------------------------------ */
 /* Device field primitives on arrays (op: 0 fe_mul, 1 fe_add, 2 fe_sub, 3 sc_mul, 4 fe_inv,

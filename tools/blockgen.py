@@ -71,10 +71,13 @@ def _der_sig(r: int, s: int) -> bytes:
 
 class Network:
     """n_orgs endorsing orgs (one peer identity each) + n_clients client identities + one identity that is NOT in the
-    MSP table ('unknown') and one whose certificate the MSP considers invalid."""
+    MSP table ('unknown') and one whose certificate the MSP considers invalid.
+    hash_families: {mspid: "SHA2" | "SHA3"}, the SignatureHashFamily of those MSPs (others SHA2): every signature is made over the
+    digest of its signer's family, as identity.Sign does (msp/identities.go:216-224,251-280).  None: SHA-256 throughout."""
 
-    def __init__(self, n_orgs=4, n_clients=1, seed=0xB10C, channel="fabgpu-channel"):
+    def __init__(self, n_orgs=4, n_clients=1, seed=0xB10C, channel="fabgpu-channel", hash_families=None):
         self.channel = channel
+        self.hash_families = dict(hash_families or {})
         self.n_orgs = n_orgs
         K = n_orgs + n_clients + 2
         L = workload.lib()
@@ -92,6 +95,12 @@ class Network:
         self.peers_alt = [Identity(p.mspid, p.priv_index, p.xy, p.cert_pem.replace(b"\n", b"\r\n")) for p in self.peers]
         self.msp_table = self.peers + self.clients + [self.invalid_cert] + self.peers_alt        # `unknown` deliberately absent
         self.principals = ["Org%dMSP" % (i + 1) for i in range(n_orgs)]
+        # key index -> hash family of the MSP that key's identity belongs to
+        self.key_family = {i.priv_index: self.hash_families.get(i.mspid, "SHA2") for i in self.msp_table + [self.unknown]}
+
+    def digest(self, priv_index, msg: bytes) -> bytes:
+        """What identity.Sign hashes before signing: SHA-256 or SHA3-256 per the signer's MSP family."""
+        return (hashlib.sha3_256 if self.key_family.get(priv_index) == "SHA3" else hashlib.sha256)(msg).digest()
 
     def policies_for(self, n_endorsements):
         """(nodes, {namespace: root}): CHAINCODE wants n_endorsements of the orgs, STRICT_NAMESPACE one more; UNKNOWN_NAMESPACE has no entry."""
@@ -179,7 +188,7 @@ def build_block(net: Network, n_tx: int, n_endorsements: int = 3, faults=None, s
     # ---- phase 2: sign endorsements, assemble payloads, sign payloads ---------------------------------------------
     def sign_all(msgs, keys):
         n = len(msgs)
-        dig = np.frombuffer(b"".join(hashlib.sha256(m).digest() for m in msgs), np.uint8).reshape(n, 32).copy()
+        dig = np.frombuffer(b"".join(net.digest(k, m) for m, k in zip(msgs, keys)), np.uint8).reshape(n, 32).copy()
         r = np.zeros((n, 32), np.uint8); s = np.zeros((n, 32), np.uint8)
         kidx = np.array(keys, np.int32)
         L.siggen_sign_batch(net.priv.ctypes.data_as(ctypes.c_void_p), kidx.ctypes.data_as(ctypes.c_void_p), dig.ctypes.data_as(ctypes.c_void_p),
